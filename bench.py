@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- the hot path of piplib-b200 on BASELINE.json's headline configuration.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--workload NAME]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--workload NAME] [--dump-outputs DIR]
   python bench.py --impl reference ...      (the reference's own CPU path, all host cores)
 
 A "step" is one pass of the solver over one batch of B synthetic problems per GPU (weak
@@ -13,8 +13,20 @@ scaling: every rank solves its own B problems; no data-path collective exists, S
 The workload is configs[1] of BASELINE.json: ~16 unknowns x 24 constraints, 3 parameters
 (workloads/synth.py: loopnest16x24p3), data = synthetic.  Inputs (4 GB per 10^6 problems) are
 far larger than L2, so no explicit L2 flush is needed between steps.
+
+--dump-outputs DIR writes what the timed calls returned in their last step as DIR/<name>.npy (float64; a
+64-bit integer array as <name>_hi = signed upper 32 bits and <name>_lo = lower 32 bits, both exact), so
+that two builds can be compared output for output on the same seeded inputs:
+  status, hash_*                 the device-resident job (the headline value): per-problem status, quast hash
+  e2e_status, e2e_hash_*         pip_solve_dense_dp on page-locked caller buffers
+  e2e_ser_index, e2e_ser_len,    the serialised quasts of a fixed seeded sample of problems (indices, words per
+  e2e_ser_words_*                problem, the words one after the other)
+  batch_api_status               pip_solve_batch_dp on the first problems of the batch
+  config4_status, config4_cells_*  the large tableau (kind, p1, p2 per cell)
+Above DUMP_PROBLEMS problems per-problem arrays hold a fixed seeded sample, listed in problem_index.
 """
 import argparse
+import atexit
 import json
 import multiprocessing as mp
 import os
@@ -34,6 +46,31 @@ from workloads import synth  # noqa: E402
 
 METRIC = "problems_per_sec"
 UNIT = "problems/s"
+# --dump-outputs budget, 64 MiB in all: 56 bytes per dumped problem (4 per-problem arrays, 48 bytes as float64
+# halves, + problem_index) = 56 MB at DUMP_PROBLEMS, 4 MiB of serialised-quast words, ~0.8 MB batch API + config 4
+DUMP_PROBLEMS = 1000000        # per-problem arrays up to this many problems are dumped whole
+DUMP_SER_PROBLEMS = 512        # problems whose serialised quasts are dumped ...
+DUMP_SER_WORDS = 1 << 18       # ... as long as their words fit in this many
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(path, arrays):
+    """arrays: name -> integer array; writes float64 .npy files (64-bit integers split in exact halves)"""
+    files = {}
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        if a.dtype.itemsize == 8:
+            v = a.view(np.int64)
+            files[name + "_hi"] = (v >> 32).astype(np.float64)
+            files[name + "_lo"] = (v & 0xffffffff).astype(np.float64)
+        else:
+            files[name] = a.astype(np.float64)
+    total = sum(f.nbytes for f in files.values())
+    if total > DUMP_LIMIT:
+        raise SystemExit("bench.py: --dump-outputs: %d bytes exceed the %d-byte limit" % (total, DUMP_LIMIT))
+    os.makedirs(path, exist_ok=True)
+    for name, f in files.items():
+        np.save(os.path.join(path, name + ".npy"), f)
 
 
 def peaks():
@@ -101,7 +138,7 @@ class ClockSampler(threading.Thread):
 from oracle.cpu_arm import cpu_arm, same_answers, usable_cores  # noqa: E402
 
 
-def large_tableau_line(pk, pk_src, n=4096, reps=2, cpu=True):
+def large_tableau_line(pk, pk_src, n=4096, reps=2, cpu=True, outputs=None):
     """BASELINE config 4 (the HBM-bound kernel of the path): one n x (n+1) int64 tableau solved by the
     whole grid, cooperative launch, CUDA events inside the library.  Algorithmic bytes per pivot =
     16*R*C + 8*C + 8*R (SURVEY.md 8d, dense figure).  Refuses to report unless the cells equal the ones
@@ -117,6 +154,9 @@ def large_tableau_line(pk, pk_src, n=4096, reps=2, cpu=True):
     if st != g["status"] or cells != g["cells"] or info["pivots"] != g["pivots"]:
         raise SystemExit("bench.py: config 4: the %d x %d tableau's answer differs from the reference's -- "
                          "refusing to report" % (n, n + 1))
+    if outputs is not None:
+        outputs["config4_status"] = np.asarray([st], dtype=np.int32)
+        outputs["config4_cells"] = np.asarray(cells, dtype=np.int64).reshape(-1, 3)
     piv = max(1, info["pivots"])
     R, C = n - 1, n + 1
     alg = (16.0 * R * C + 8.0 * C + 8.0 * R) * piv
@@ -180,13 +220,19 @@ def main():
     ap.add_argument("--no-large", action="store_true", help="skip the config-4 large-tableau measurement")
     ap.add_argument("--check", type=int, default=65536,
                     help="problems of every rank's own range cross-checked against the reference before timing")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the timed calls returned in their last step to DIR/<name>.npy (rank 0)")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs dumps the GPU path (--impl ours)")
 
     rank, world, local = pdist.env_rank()
     cores = len(usable_cores())
     bg, opts = synth.bignum(a.workload), synth.options(a.workload)
     W = max(a.warmup, 0)
-    K = max(a.steps, 1)
+    K = a.steps
     B = a.batch
     if a.total:
         B = (a.total + world - 1) // world
@@ -279,6 +325,7 @@ def main():
     sampler = ClockSampler(local)
     if rank == 0:
         sampler.start()
+        atexit.register(sampler.stop)        # no nvidia-smi left running if the timed region raises
     barrier()
     t0 = time.perf_counter()
     dev_ms, launches = 0.0, 0
@@ -289,7 +336,10 @@ def main():
         launches += stats.launches
     barrier()
     wall_ms = 1e3 * (time.perf_counter() - t0)
-    status, _ = db.results(False)
+    outputs = {} if a.dump_outputs and rank == 0 else None
+    status, hashes = db.results(outputs is not None)
+    if outputs is not None:
+        outputs["status"], outputs["hash"] = status, hashes
     pivots_step = int(stats.pivots)
     elem_step = int(stats.elem_updates)
     cells_step = int(stats.cells)
@@ -319,6 +369,14 @@ def main():
         s2 = api.last_stats()
         h2d_b, d2h_b = int(s2.h2d_bytes), int(s2.d2h_bytes)
         api.unpin(dom), api.unpin(ctx)
+        if outputs is not None:
+            outputs["e2e_status"], outputs["e2e_hash"] = res["status"], res["hashes"]
+            idx = np.sort(np.random.default_rng(a.seed).choice(B, size=min(B, DUMP_SER_PROBLEMS), replace=False))
+            idx = idx[np.cumsum(res["ser_len"][idx]) <= DUMP_SER_WORDS]
+            outputs["e2e_ser_index"] = idx.astype(np.int32)
+            outputs["e2e_ser_len"] = res["ser_len"][idx].astype(np.int32)
+            outputs["e2e_ser_words"] = np.concatenate(
+                [res["ser"][res["ser_off"][i]:res["ser_off"][i] + res["ser_len"][i]] for i in idx])
     if rank == 0:
         sampler.stop()
 
@@ -391,7 +449,7 @@ def main():
                                         "buffers": "pageable caller arrays: host thread pool narrows into / widens "
                                                    "out of pinned staging"}
         if world == 1 and not a.no_large:
-            line["config4_large_tableau"] = large_tableau_line(pk, pk_src)
+            line["config4_large_tableau"] = large_tableau_line(pk, pk_src, outputs=outputs)
         if world == 1 and not a.no_e2e:
             # the entry point north_star names: pip_solve_batch_dp (PipMatrix objects in, malloc'd PipQuast trees
             # out), on a bounded slice (building the matrices through ctypes is the slow part, outside the timing)
@@ -399,6 +457,8 @@ def main():
             sec, st_b = api.time_solve_batch(dom[:nb], ctx[:nb], bg, **opts)
             if res is not None and not np.array_equal(np.where(st_b == 1, 0, st_b), np.where(res["status"][:nb] == 1, 0, res["status"][:nb])):
                 raise SystemExit("bench.py: pip_solve_batch_dp and pip_solve_dense_dp disagree")
+            if outputs is not None:
+                outputs["batch_api_status"] = st_b
             line["batch_api"] = {"value": nb / sec, "unit": UNIT, "problems": nb,
                                  "api": "pip_solve_batch_dp: PipMatrix objects in, PipQuast trees out (host decode, malloc per node)"}
         if world == 1:
@@ -414,7 +474,17 @@ def main():
                                     "sample": "first %d problems of the batch, one process per core, "
                                               "pip_solve loop; statuses and quast hashes equal to the timed "
                                               "GPU run's" % sample}
+        if outputs is not None:
+            if B > DUMP_PROBLEMS:
+                keep = np.sort(np.random.default_rng(a.seed + 1).choice(B, size=DUMP_PROBLEMS, replace=False))
+                outputs["problem_index"] = keep.astype(np.int32)
+                for k in ("status", "hash", "e2e_status", "e2e_hash"):
+                    if k in outputs:
+                        outputs[k] = outputs[k][keep]
         print(json.dumps(line))
+        sys.stdout.flush()
+        if outputs is not None:
+            dump_outputs(a.dump_outputs, outputs)
     if world > 1:
         dist.barrier()
         dist.destroy_process_group()

@@ -18,7 +18,6 @@ import numpy as np
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 REF_SO = os.path.join(HERE, "_ref", "libpipref.so")
-EXAMPLE_DP = os.path.join(HERE, "_ref", "example_dp")       # reference example/example.c linked with OUR library
 REF_BIG_SO = os.path.join(HERE, "_ref", "libpipref_big.so")     # same sources, SOL_SIZE / MAXCOL raised by -D
 PORT_SO = os.path.join(HERE, "libpiporacle.so")
 
@@ -35,7 +34,7 @@ def build(ref=True, port=True):
     if port:
         targets.append("libpiporacle.so")
     if ref and os.path.isdir("/root/reference/source"):
-        targets += ["ref", "refbig", "example"]
+        targets += ["ref", "refbig"]
     if targets:
         subprocess.check_call(["make", "-s", "-C", HERE] + targets)
 

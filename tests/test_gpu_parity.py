@@ -559,13 +559,13 @@ def test_one_call_over_several_gpus(api, port):
         del os.environ["PIPLIB_B200_CHUNK"]
 
 
-def test_reference_example_program_runs_on_our_library(api):
-    """the reference's own caller (example/example.c, compiled UNCHANGED against include/ and linked with
-    libpiplib_dp.so: oracle/_ref/example_dp, oracle/Makefile `example`) replays every example/*.pip and its
-    option variants: stdout must be the reference's .ll text (prompts, echoed matrices, pip_quast_print)"""
+def test_reference_example_program_runs_on_our_library(api, tmp_path):
+    """the reference's own caller (example/example.c: tests/fixtures/example.c compiled against include/ and
+    linked with libpiplib_dp.so) replays every example/*.pip and its option variants: stdout must be the
+    reference's .ll text (prompts, echoed matrices, pip_quast_print)"""
     import subprocess
-    if not os.path.exists(po.EXAMPLE_DP):
-        pytest.skip("oracle/_ref/example_dp not built")
+    from test_cabi import build_example
+    exe = build_example(api.LIB_PATH, tmp_path)
     flags = {"Maximize": "Maximize", "Urs_parms": "Urs_parms", "Urs_unknowns": "Urs_unknowns", "Compute_dual": "Dual"}
 
     def mat(shape, rows):
@@ -580,7 +580,7 @@ def test_reference_example_program_runs_on_our_library(api):
                 text += word + "\n"
         if not c["opts"].get("Nq", 1):
             text += "Rational\n"
-        r = subprocess.run([po.EXAMPLE_DP], input=text, capture_output=True, text=True, timeout=120)
+        r = subprocess.run([exe], input=text, capture_output=True, text=True, timeout=120)
         if r.returncode != 0 or po.strip_ws_lines(r.stdout) != po.strip_ws_lines(c["golden_ll"]):
             bad.append((c["name"], r.returncode, r.stderr[-200:]))
         checked += 1
