@@ -13,7 +13,8 @@
  *   pip_solve_dense_dp        pip_solve_batch_dp for a batch whose problems share one shape,
  *                             given as two dense int64 arrays (no PipMatrix objects); returns
  *                             cells or a hash per problem.  This is the bulk path used by
- *                             bench.py (host buffers in, host buffers out).
+ *                             bench.py (host buffers in, host buffers out); it also reads and
+ *                             writes caller arrays in device memory.
  *   pip_device_*              the same batch with inputs/outputs resident in device memory
  *                             (kernel-only timing; pointers are CUdeviceptr values as integers).
  *   pip_quast_serialize_dp    PipQuast -> int64 stream (test/interop helper).
@@ -101,14 +102,28 @@ void pip_cells_simplify_dp(PipCell_dp *cells, int *ncells);
 void pip_cells_bind_dp(const PipCell_dp *cells, int ncells);
 
 /* Dense batch through the pip_solve_dp path: dom is [n][dom_rows][dom_cols] (PolyLib rows),
- * ctx is [n][ctx_rows][ctx_cols] or NULL (has_ctx=0).  Host buffers in, host buffers out:
+ * ctx is [n][ctx_rows][ctx_cols] or NULL (has_ctx=0):
  *   status[i]  as above
  *   hashes[i]  (optional) hash of the serialised quast words (pip_hash_word: a sum of mixed (word, index) pairs; the function tests/ and
  *              oracle/ apply to the reference's trees); 0 when status[i] is fatal
  *   ser        (optional) the serialised quasts: problem i occupies
  *              ser[ser_off[i] .. ser_off[i] + ser_len[i]); spans are packed without gaps but, as
  *              chunks of the batch finish in any order, not in problem order.  ser_off has n+1
- *              entries, ser_off[n] = words used/needed; returns -2 when ser_cap is too small. */
+ *              entries, ser_off[n] = words used/needed; returns -2 when ser_cap is too small.
+ * Returns 0, -2 (above), -3 (device buffers refused, below) or -1 (a CUDA or system error).
+ *
+ * Buffers may be host memory (pageable or page-locked, see pip_pin_buffer_dp) or device memory (cudaMalloc,
+ * torch CUDA tensors; managed memory counts as host memory).  The inputs (dom and ctx) and the outputs
+ * (status, hashes, ser, ser_off, ser_len: the non-NULL ones) are placed independently:
+ *   device inputs   the rows are converted where they are; they never cross PCIe
+ *   device outputs  every output, ser_off[n] included, is written in device memory, by the device
+ * Device-resident buffers run on the device that owns them, whatever pip_set_device_dp / pip_set_devices_dp
+ * say.  The call returns -3, before anything is written, when the device-resident arrays are on different
+ * devices, when only one of dom / ctx is device-resident or only some of the outputs are, or when
+ * device-resident buffers meet an option the host decoder serves (Simplify; Compute_dual with Nq = 0).
+ * Ordering: the work that writes device inputs (or last used device outputs) must be complete when the call
+ * is made -- the library runs on CUDA streams of its own -- and device outputs are complete when it returns.
+ * The call is host-synchronous in every case. */
 int pip_solve_dense_dp(long long n, int dom_rows, int dom_cols, const long long *dom,
                        int has_ctx, int ctx_rows, int ctx_cols, const long long *ctx,
                        int bignum, const PipOptions_dp *options,

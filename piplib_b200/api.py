@@ -314,25 +314,76 @@ def traiter_batch(cases):
     return out
 
 
+def _ptr(a):
+    """address of a numpy array, or of a torch tensor's data (host or device memory)"""
+    return C.c_void_p(a.data_ptr()) if hasattr(a, "data_ptr") else a.ctypes.data_as(C.c_void_p)
+
+
+def _ready(*arrays):
+    """the library works on CUDA streams of its own: whatever torch queued on the current stream of a device that
+    holds one of the arrays (producing the inputs, clearing the outputs) must be complete before the call"""
+    devices = {a.device for a in arrays if getattr(a, "is_cuda", False)}
+    if devices:
+        import torch
+        for d in devices:
+            torch.cuda.current_stream(d).synchronize()
+
+
+class _HostArrays:
+    """solve_dense on numpy arrays (pageable or page-locked host memory)"""
+
+    def input(self, a):
+        return np.ascontiguousarray(a, dtype=np.int64)
+
+    def zeros(self, n, dtype):
+        return np.zeros(n, dtype=np.uint64 if dtype == "u64" else dtype)
+
+    def empty(self, n):
+        return np.empty(n, dtype=np.int64)
+
+
+class _CudaTensors:
+    """solve_dense on torch CUDA tensors: the library reads the rows and writes the results in device memory,
+    on the device that holds them.  Hashes come back as int64 tensors holding the uint64 bits."""
+
+    def __init__(self, like):
+        import torch
+        self.torch, self.device = torch, like.device
+
+    def input(self, a):
+        if not getattr(a, "is_cuda", False) or a.device != self.device:
+            raise ValueError("solve_dense: dom and ctx must both be CUDA tensors on one device, or both host arrays")
+        return a.to(self.torch.int64).contiguous()
+
+    def zeros(self, n, dtype):
+        return self.torch.zeros(n, dtype=self.torch.int32 if dtype == np.int32 else self.torch.int64, device=self.device)
+
+    def empty(self, n):
+        return self.torch.empty(n, dtype=self.torch.int64, device=self.device)
+
+
 def solve_dense(dom, ctx, bignum=-1, want_hashes=True, want_ser=False, ser_cap_hint=None, out=None, **opts):
-    """dom: [n, rows, cols] int64 (host); ctx: [n, rows, cols] or None.
-    Returns dict(status, hashes, ser, ser_off)."""
+    """dom: [n, rows, cols] int64; ctx: [n, rows, cols] or None.  Host arrays (numpy), or torch CUDA tensors:
+    these are read and the results written in GPU memory, and the results are CUDA tensors (status int32,
+    hashes / ser / ser_off / ser_len int64; hashes hold the uint64 bits).
+    Returns dict(status, hashes, ser, ser_off, ser_len)."""
     L = lib()
-    dom = np.ascontiguousarray(dom, dtype=np.int64)
+    B = _CudaTensors(dom) if getattr(dom, "is_cuda", False) else _HostArrays()
+    dom = B.input(dom)
     n, dr, dc = dom.shape
     if ctx is None:
         has, cr, cc, cp = 0, 0, 0, None
     else:
-        ctx = np.ascontiguousarray(ctx, dtype=np.int64)
+        ctx = B.input(ctx)
         has, cr, cc = 1, ctx.shape[1], ctx.shape[2]
-        cp = ctx.ctypes.data_as(C.c_void_p)
+        cp = _ptr(ctx)
     # `out` = the dict returned by an earlier call of the same shape: its (caller-owned) result
     # buffers are reused instead of allocating and page-faulting gigabytes again
     reuse = out is not None and out["status"].shape[0] == n
-    status = out["status"] if reuse else np.zeros(n, dtype=np.int32)
+    status = out["status"] if reuse else B.zeros(n, np.int32)
     hashes = None
     if want_hashes:
-        hashes = out["hashes"] if reuse and out.get("hashes") is not None else np.zeros(n, dtype=np.uint64)
+        hashes = out["hashes"] if reuse and out.get("hashes") is not None else B.zeros(n, "u64")
     o = make_options(**opts)
     ser = ser_off = ser_len = None
     cap = 0
@@ -341,25 +392,29 @@ def solve_dense(dom, ctx, bignum=-1, want_hashes=True, want_ser=False, ser_cap_h
             ser, ser_off, ser_len = out["ser"], out["ser_off"], out["ser_len"]
             cap = ser.shape[0]
         else:
-            ser_off = np.zeros(n + 1, dtype=np.int64)
-            ser_len = np.zeros(n, dtype=np.int64)
+            ser_off = B.zeros(n + 1, np.int64)
+            ser_len = B.zeros(n, np.int64)
             cap = (ser_cap_hint or 448) * n + 1024
-            ser = np.empty(cap, dtype=np.int64)
+            ser = B.empty(cap)
     while True:
-        rc = L.pip_solve_dense_dp(C.c_longlong(n), dr, dc, dom.ctypes.data_as(C.c_void_p), has, cr, cc, cp,
-                                  int(bignum), C.byref(o), status.ctypes.data_as(C.c_void_p),
-                                  hashes.ctypes.data_as(C.c_void_p) if want_hashes else None,
-                                  ser.ctypes.data_as(C.c_void_p) if want_ser else None,
+        _ready(dom, ctx, status, hashes, ser, ser_off, ser_len)
+        rc = L.pip_solve_dense_dp(C.c_longlong(n), dr, dc, _ptr(dom), has, cr, cc, cp,
+                                  int(bignum), C.byref(o), _ptr(status),
+                                  _ptr(hashes) if want_hashes else None,
+                                  _ptr(ser) if want_ser else None,
                                   C.c_longlong(cap),
-                                  ser_off.ctypes.data_as(C.c_void_p) if want_ser else None,
-                                  ser_len.ctypes.data_as(C.c_void_p) if want_ser else None)
+                                  _ptr(ser_off) if want_ser else None,
+                                  _ptr(ser_len) if want_ser else None)
         if rc == -2:
-            was_pinned = reuse and out.get("ser") is ser
+            was_pinned = reuse and out.get("ser") is ser and isinstance(ser, np.ndarray)
             cap = int(ser_off[n]) + 16
-            ser = np.empty(cap, dtype=np.int64)
+            ser = ser.new_empty(cap) if hasattr(ser, "new_empty") else np.empty(cap, dtype=np.int64)
             if was_pinned:
                 pin(ser)
             continue
+        if rc == -3:
+            raise RuntimeError("pip_solve_dense_dp refused the device-resident buffers (-3): they are on different "
+                               "devices, mix host and device memory, or meet an option the host decoder serves")
         if rc != 0:
             raise RuntimeError("pip_solve_dense_dp failed: %d" % rc)
         break

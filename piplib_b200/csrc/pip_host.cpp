@@ -1163,13 +1163,27 @@ void emit_chunk_staged(size_t first, size_t n, const pip_i64 *words, const int *
   });
 }
 
-bool is_pinned(const void *p)
+/* where a caller buffer lives; managed memory is treated as pageable host memory */
+enum MemKind { MEM_PAGEABLE, MEM_PINNED, MEM_DEVICE };
+MemKind mem_kind(const void *p, int *device = nullptr)
 {
-  if (!p) return false;
+  if (!p) return MEM_PAGEABLE;
   cudaPointerAttributes a;
-  if (cudaPointerGetAttributes(&a, p) != cudaSuccess) { cudaGetLastError(); return false; }
-  return a.type == cudaMemoryTypeHost;
+  if (cudaPointerGetAttributes(&a, p) != cudaSuccess) { cudaGetLastError(); return MEM_PAGEABLE; }
+  if (a.type == cudaMemoryTypeDevice) {
+    if (device) *device = a.device;
+    return MEM_DEVICE;
+  }
+  return a.type == cudaMemoryTypeHost ? MEM_PINNED : MEM_PAGEABLE;
 }
+bool is_pinned(const void *p) { return mem_kind(p) == MEM_PINNED; }
+
+/* the calling thread's current device is the caller's: the dense path selects the devices it runs on */
+struct KeepCurrentDevice {
+  int saved = -1;
+  KeepCurrentDevice() { if (cudaGetDevice(&saved) != cudaSuccess) { cudaGetLastError(); saved = -1; } }
+  ~KeepCurrentDevice() { if (saved >= 0) cudaSetDevice(saved); }
+};
 
 std::mutex g_dense_mu;                  /* one dense call at a time per process (it is parallel inside) */
 /* One lane at a time per device and direction on the PCIe link: lanes that all upload, then all solve, then
@@ -1238,28 +1252,60 @@ int pip_solve_dense_dp(long long n, int dom_rows, int dom_cols, const long long 
 {
   if (n <= 0) return 0;
   std::lock_guard<std::mutex> dense_guard(g_dense_mu);
+  KeepCurrentDevice keep_device;
   try {
     const double t0 = wall();
     DenseArgs A = {n, dom_rows, dom_cols, dom, has_ctx, ctx_rows, ctx_cols, ctx, bignum,
                    options ? *options : DEFAULT_OPTIONS};
+    /* Caller arrays in device memory: the inputs are converted where they are and the results are written
+     * there.  Every device-resident array must be on one device, and the inputs and the outputs each go
+     * wholly one way or the other; nothing has been written when such a call is refused. */
+    const bool ctx_used = has_ctx && ctx_rows > 0;
+    int owner = -1;
+    bool other_device = false;
+    auto on_device = [&](const void *p) {
+      int d = -1;
+      if (mem_kind(p, &d) != MEM_DEVICE) return false;
+      if (owner >= 0 && d != owner) other_device = true;
+      owner = d;
+      return true;
+    };
+    const bool in_device = on_device(dom);
+    const bool ctx_device = ctx_used && on_device(ctx);
+    int nout = 0, nout_device = 0;
+    for (const void *p : {(const void *)status, (const void *)hashes, (const void *)ser, (const void *)ser_off, (const void *)ser_len})
+      if (p) { nout++; nout_device += on_device(p) ? 1 : 0; }
+    const bool out_device = nout_device > 0;
+    const bool host_decoder = A.opt.Simplify || (A.opt.Compute_dual && !A.opt.Nq);
+    if (other_device || (ctx_used && ctx_device != in_device) || (out_device && nout_device != nout) ||
+        ((in_device || out_device) && host_decoder))
+      return -3;
     std::vector<int> devices;
     {
       std::lock_guard<std::mutex> g(g_devices_mu);
       devices = g_devices;
     }
     if (devices.empty()) devices.push_back(pip_engine_device());
+    if (owner >= 0) devices.assign(1, owner);          /* device-resident arrays: the device that owns them */
     const bool keep = ser != nullptr && ser_off != nullptr;
     /* decode on the GPU unless the host-only Simplify post-pass is wanted (PIPLIB_B200_HOST_DECODE=1
-     * forces the host decoder, for A/B tests) */
-    const bool device_decode = !A.opt.Simplify && !(A.opt.Compute_dual && !A.opt.Nq) &&
-                               getenv("PIPLIB_B200_HOST_DECODE") == nullptr;
-    /* Caller buffers in pinned (page-locked) memory are moved by DMA alone: the raw PolyLib rows go up as
-     * they are and tab_Matrix2Tableau runs on the device (pip_convert_kernel); the serialised quasts come
-     * down straight into the caller's stream.  Pageable buffers are converted (narrowed to int8 / int32)
-     * by the host pool into pinned staging, and widened out of it. */
-    const bool in_pinned = device_decode && is_pinned(dom) && (!has_ctx || !ctx_rows || is_pinned(ctx)) &&
+     * forces the host decoder, for A/B tests, except for device-resident arrays, which it cannot write) */
+    const bool device_decode = !host_decoder && (getenv("PIPLIB_B200_HOST_DECODE") == nullptr || in_device || out_device);
+    /* Input stage.  Caller rows in device memory are converted in place (pip_convert_kernel reads them where
+     * they are).  Caller buffers in pinned (page-locked) memory are moved by DMA alone: the raw PolyLib rows
+     * go up as they are and tab_Matrix2Tableau runs on the device.  Pageable buffers are converted (narrowed
+     * to int8 / int32) by the host pool into pinned staging. */
+    enum InRoute { IN_HOST_CONVERT, IN_DMA_CONVERT, IN_DEVICE_CONVERT };
+    const bool in_pinned = device_decode && is_pinned(dom) && (!ctx_used || is_pinned(ctx)) &&
                            getenv("PIPLIB_B200_HOST_CONVERT") == nullptr;
-    const bool out_pinned = device_decode && keep && is_pinned(ser) && getenv("PIPLIB_B200_STAGED_OUT") == nullptr;
+    const InRoute in_route = in_device ? IN_DEVICE_CONVERT : in_pinned ? IN_DMA_CONVERT : IN_HOST_CONVERT;
+    /* Output stage.  Device-resident outputs are written on the device (one device-to-device copy of the
+     * chunk's words, pip_emit_device_kernel for the per-problem arrays); a pinned stream receives the words
+     * straight from the device; pageable outputs are staged through pinned scratch and widened out of it. */
+    enum OutRoute { OUT_STAGED, OUT_PINNED_DMA, OUT_DEVICE };
+    const bool out_pinned = device_decode && keep && is_pinned(ser) &&
+                            getenv("PIPLIB_B200_STAGED_OUT") == nullptr;
+    const OutRoute out_route = out_device ? OUT_DEVICE : out_pinned ? OUT_PINNED_DMA : OUT_STAGED;
 
     /* chunk schedule: full chunks of CH problems, with a geometric ramp at both ends (CH/8, CH/4,
      * CH/2) so that the GPU starts after one small transfer and the last copy-out is short */
@@ -1321,16 +1367,17 @@ int pip_solve_dense_dp(long long n, int dom_rows, int dom_cols, const long long 
      * chunk queue.  Measured on a box whose link does 55 GB/s each way: no gain (the upload is not what bounds
      * the call), so it is off; a box with a slower link may want it. */
     size_t host_lanes = 0;
-    if (in_pinned) {
+    if (in_route == IN_DMA_CONVERT) {
       if (const char *hv = getenv("PIPLIB_B200_HOST_LANES")) host_lanes = (size_t)std::max(0, atoi(hv));
       host_lanes = std::min<size_t>(host_lanes, lanes > 1 ? lanes - 1 : 0);
     }
     auto worker_main = [&](size_t w) {
       try {
         const int device = devices[w / lanes];
-        const bool lane_dma = in_pinned && (w % lanes) >= host_lanes;
-        const size_t nthreads = (in_pinned && !lane_dma) ? std::max<size_t>(1, host_threads() / std::max<size_t>(1, host_lanes * devices.size()))
-                                                          : nthreads_default;
+        const InRoute lane_in = (in_route == IN_DMA_CONVERT && (w % lanes) < host_lanes) ? IN_HOST_CONVERT : in_route;
+        const size_t nthreads = (in_route == IN_DMA_CONVERT && lane_in == IN_HOST_CONVERT)
+                                    ? std::max<size_t>(1, host_threads() / std::max<size_t>(1, host_lanes * devices.size()))
+                                    : nthreads_default;
         PipEngine &E = PipEngine::at(device, (int)(w % lanes));
         cudaStream_t s = E.stream();
         pip_cuda_check(cudaSetDevice(device), "cudaSetDevice");
@@ -1349,23 +1396,29 @@ int pip_solve_dense_dp(long long n, int dom_rows, int dom_cols, const long long 
           PipProblem uniform;
           struct WidenCtx { PipConvertArgs a; void *pool64; } wc;
           wc.pool64 = nullptr;
-          if (lane_dma) {
-            /* ---- DMA the raw rows up, convert on the device ---- */
+          if (lane_in != IN_HOST_CONVERT) {
+            /* ---- convert the raw rows on the device: the caller's rows where they are, or a DMA'd copy ---- */
             const size_t dwords = (size_t)A.dr * A.dc, cwords = CS.has_ctx ? (size_t)A.cr * A.cc : 0;
-            pip_i64 *d_dom = (pip_i64 *)E.device_scratch(0, std::max<size_t>(cn * dwords * 8, 8));
-            pip_i64 *d_ctx = (pip_i64 *)E.device_scratch(1, std::max<size_t>(cn * cwords * 8, 8));
+            const pip_i64 *d_dom, *d_ctx;
+            if (lane_in == IN_DEVICE_CONVERT) {
+              d_dom = A.dom + C.first * dwords;
+              d_ctx = cwords ? A.ctx + C.first * cwords : nullptr;
+            } else {
+              pip_i64 *up_dom = (pip_i64 *)E.device_scratch(0, std::max<size_t>(cn * dwords * 8, 8));
+              pip_i64 *up_ctx = (pip_i64 *)E.device_scratch(1, std::max<size_t>(cn * cwords * 8, 8));
+              std::lock_guard<std::mutex> link(g_h2d_mu[device]);
+              if (dwords) pip_cuda_check(cudaMemcpyAsync(up_dom, A.dom + C.first * dwords, cn * dwords * 8, cudaMemcpyHostToDevice, s), "H2D domain rows");
+              if (cwords) pip_cuda_check(cudaMemcpyAsync(up_ctx, A.ctx + C.first * cwords, cn * cwords * 8, cudaMemcpyHostToDevice, s), "H2D context rows");
+              pip_cuda_check(cudaEventRecord(copied, s), "cudaEventRecord");
+              pip_cuda_check(cudaEventSynchronize(copied), "wait for the upload");      /* (not for the kernels behind it) */
+              lane_stats[w].h2d_bytes += cn * (dwords + cwords) * 8;
+              d_dom = up_dom; d_ctx = up_ctx;
+            }
             const long long stride = 2ll * A.dr * CS.width + 2ll * CS.cr * CS.cwidth;
             void *d_pool = E.device_scratch(2, std::max<size_t>((size_t)cn * stride * 4, 8));
             unsigned char *d_pd = (unsigned char *)E.device_scratch(3, cn * sizeof(PipProblem) + 64);
             int *d_dims = (int *)(d_pd + cn * sizeof(PipProblem));
             int *h_dims = (int *)E.pinned_scratch(0, 64);
-            {
-              std::lock_guard<std::mutex> link(g_h2d_mu[device]);
-              if (dwords) pip_cuda_check(cudaMemcpyAsync(d_dom, A.dom + C.first * dwords, cn * dwords * 8, cudaMemcpyHostToDevice, s), "H2D domain rows");
-              if (cwords) pip_cuda_check(cudaMemcpyAsync(d_ctx, A.ctx + C.first * cwords, cn * cwords * 8, cudaMemcpyHostToDevice, s), "H2D context rows");
-              pip_cuda_check(cudaEventRecord(copied, s), "cudaEventRecord");
-              pip_cuda_check(cudaEventSynchronize(copied), "wait for the upload");      /* (not for the kernels behind it) */
-            }
             pip_cuda_check(cudaMemsetAsync(d_dims, 0, 16, s), "memset dims");
             PipConvertArgs &ca = wc.a;
             ca.s = CS; ca.dom = d_dom; ca.ctx = d_ctx; ca.n = (long long)cn; ca.stride = stride;
@@ -1389,7 +1442,6 @@ int pip_solve_dense_dp(long long n, int dom_rows, int dom_cols, const long long 
               }
               return w->pool64;
             };
-            lane_stats[w].h2d_bytes += cn * (dwords + cwords) * 8;
           } else {
             /* ---- convert on the host (narrowing) into pinned staging ---- */
             const bool optimistic = uniform_hint.load() != 0;
@@ -1415,55 +1467,70 @@ int pip_solve_dense_dp(long long n, int dom_rows, int dom_cols, const long long 
             in.stream_out = true;
             /* other lanes keep the machine busy during this chunk's tail -- except at the end of the call */
             in.overlapped = nworkers > 1 && c + tail_chunks < nchunks;
-            in.words64 = out_pinned;
+            in.words64 = out_route == OUT_PINNED_DMA || (out_route == OUT_DEVICE && keep);
           }
           double td = wall();
           E.run(in, C.out);
           double te = wall();
           if (wc.pool64) { cudaFree(wc.pool64); wc.pool64 = nullptr; }
           if (device_decode) {
-            /* per-problem arrays: SoA on the device -> pinned scratch -> the caller's arrays */
             const PipDeviceOut &D = C.out.dev;
-            const size_t soa = cn * (sizeof(int) + sizeof(pip_u64) + 2 * sizeof(long long));
-            unsigned char *hp = (unsigned char *)E.pinned_scratch(1, soa + 64);
-            long long *h_off = (long long *)hp, *h_len = h_off + cn;
-            pip_u64 *h_hash = (pip_u64 *)(h_len + cn);
-            int *h_st = (int *)(h_hash + cn);
-            std::unique_lock<std::mutex> link(g_d2h_mu[device]);
-            pip_cuda_check(cudaMemcpyAsync(h_off, D.off, cn * 8, cudaMemcpyDeviceToHost, s), "D2H offsets");
-            pip_cuda_check(cudaMemcpyAsync(h_len, D.len, cn * 8, cudaMemcpyDeviceToHost, s), "D2H lengths");
-            pip_cuda_check(cudaMemcpyAsync(h_hash, D.hash, cn * 8, cudaMemcpyDeviceToHost, s), "D2H hashes");
-            pip_cuda_check(cudaMemcpyAsync(h_st, D.status, cn * 4, cudaMemcpyDeviceToHost, s), "D2H statuses");
-            lane_stats[w].d2h_bytes += soa;
-            if (out_pinned) {
-              /* the chunk's words are one contiguous span of int64: one DMA into the caller's stream */
-              const long long total = D.slots;
-              const long long base = cursor.fetch_add(total);
-              const bool fits = base + total <= ser_cap;
-              if (fits && total) {
-                pip_cuda_check(cudaMemcpyAsync(ser + base, D.words, (size_t)total * 8, cudaMemcpyDeviceToHost, s), "D2H quasts");
-                lane_stats[w].d2h_bytes += (size_t)total * 8;
+            if (out_route == OUT_DEVICE) {
+              /* the chunk's words (one contiguous span of int64) and its per-problem arrays stay on the device */
+              long long base = 0;
+              if (keep) {
+                base = cursor.fetch_add(D.slots);
+                if (D.slots && base + D.slots <= ser_cap)
+                  pip_cuda_check(cudaMemcpyAsync(ser + base, D.words, (size_t)D.slots * 8, cudaMemcpyDeviceToDevice, s), "D2D quasts");
               }
-              pip_cuda_check(cudaStreamSynchronize(s), "sync after D2H");
-              link.unlock();
-              for (size_t i = 0; i < cn; i++) {
-                const int s0 = h_st[i];
-                status[C.first + i] = PIP_STATUS_IS_FINAL(s0) ? s0 : PIP_ST_CAPACITY;
-                ser_off[C.first + i] = base + h_off[i];
-                if (ser_len) ser_len[C.first + i] = h_len[i] & ~PIP_LEN_NARROW;
-              }
-              if (hashes) memcpy(hashes + C.first, h_hash, cn * 8);
+              pip_cuda_check(pip_launch_emit_device(D.status, D.hash, D.off, D.len, (long long)cn, base, status + C.first,
+                                                    hashes ? hashes + C.first : nullptr,
+                                                    keep ? ser_off + C.first : nullptr,
+                                                    keep && ser_len ? ser_len + C.first : nullptr, s), "emit kernel");
+              pip_cuda_check(cudaStreamSynchronize(s), "sync after emit");
             } else {
-              pip_i64 *h_words = nullptr;
-              if (keep && D.slots) {
-                h_words = (pip_i64 *)E.pinned_scratch(2, (size_t)D.slots * 8);
-                pip_cuda_check(cudaMemcpyAsync(h_words, D.words, (size_t)D.slots * 8, cudaMemcpyDeviceToHost, s), "D2H quasts");
-                lane_stats[w].d2h_bytes += (size_t)D.slots * 8;
+              /* per-problem arrays: SoA on the device -> pinned scratch -> the caller's arrays */
+              const size_t soa = cn * (sizeof(int) + sizeof(pip_u64) + 2 * sizeof(long long));
+              unsigned char *hp = (unsigned char *)E.pinned_scratch(1, soa + 64);
+              long long *h_off = (long long *)hp, *h_len = h_off + cn;
+              pip_u64 *h_hash = (pip_u64 *)(h_len + cn);
+              int *h_st = (int *)(h_hash + cn);
+              std::unique_lock<std::mutex> link(g_d2h_mu[device]);
+              pip_cuda_check(cudaMemcpyAsync(h_off, D.off, cn * 8, cudaMemcpyDeviceToHost, s), "D2H offsets");
+              pip_cuda_check(cudaMemcpyAsync(h_len, D.len, cn * 8, cudaMemcpyDeviceToHost, s), "D2H lengths");
+              pip_cuda_check(cudaMemcpyAsync(h_hash, D.hash, cn * 8, cudaMemcpyDeviceToHost, s), "D2H hashes");
+              pip_cuda_check(cudaMemcpyAsync(h_st, D.status, cn * 4, cudaMemcpyDeviceToHost, s), "D2H statuses");
+              lane_stats[w].d2h_bytes += soa;
+              if (out_route == OUT_PINNED_DMA) {
+                /* the chunk's words are one contiguous span of int64: one DMA into the caller's stream */
+                const long long total = D.slots;
+                const long long base = cursor.fetch_add(total);
+                const bool fits = base + total <= ser_cap;
+                if (fits && total) {
+                  pip_cuda_check(cudaMemcpyAsync(ser + base, D.words, (size_t)total * 8, cudaMemcpyDeviceToHost, s), "D2H quasts");
+                  lane_stats[w].d2h_bytes += (size_t)total * 8;
+                }
+                pip_cuda_check(cudaStreamSynchronize(s), "sync after D2H");
+                link.unlock();
+                for (size_t i = 0; i < cn; i++) {
+                  const int s0 = h_st[i];
+                  status[C.first + i] = PIP_STATUS_IS_FINAL(s0) ? s0 : PIP_ST_CAPACITY;
+                  ser_off[C.first + i] = base + h_off[i];
+                  if (ser_len) ser_len[C.first + i] = h_len[i] & ~PIP_LEN_NARROW;
+                }
+                if (hashes) memcpy(hashes + C.first, h_hash, cn * 8);
+              } else {
+                pip_i64 *h_words = nullptr;
+                if (keep && D.slots) {
+                  h_words = (pip_i64 *)E.pinned_scratch(2, (size_t)D.slots * 8);
+                  pip_cuda_check(cudaMemcpyAsync(h_words, D.words, (size_t)D.slots * 8, cudaMemcpyDeviceToHost, s), "D2H quasts");
+                  lane_stats[w].d2h_bytes += (size_t)D.slots * 8;
+                }
+                pip_cuda_check(cudaStreamSynchronize(s), "sync after D2H");
+                link.unlock();
+                emit_chunk_staged(C.first, cn, h_words, h_st, h_hash, h_off, h_len, status, hashes, ser, ser_cap, ser_off,
+                                  ser_len, &cursor, nthreads, at);
               }
-              pip_cuda_check(cudaStreamSynchronize(s), "sync after D2H");
-              link.unlock();
-              emit_chunk_staged(C.first, cn, h_words, h_st, h_hash, h_off, h_len, status, hashes, ser, ser_cap, ser_off,
-                                ser_len, &cursor, nthreads, at);
             }
             PipBatchStats_dp &ls = lane_stats[w];
             ls.pivots += D.stats[0]; ls.cuts += D.stats[1]; ls.subsolves += D.stats[2]; ls.splits += D.stats[3];
@@ -1490,15 +1557,19 @@ int pip_solve_dense_dp(long long n, int dom_rows, int dom_cols, const long long 
     }
     for (const std::string &e : errors) if (!e.empty()) throw std::runtime_error(e);
     const long long total = cursor.load();
-    if (ser_off) ser_off[n] = total;
+    if (ser_off && out_route == OUT_DEVICE) {
+      pip_cuda_check(cudaSetDevice(owner), "cudaSetDevice");
+      pip_cuda_check(cudaMemcpy(ser_off + n, &total, sizeof total, cudaMemcpyHostToDevice), "H2D words used");
+    } else if (ser_off) ser_off[n] = total;
     if (timing) {
+      static const char *const in_name[] = {"pageable: host conversion", "pinned: DMA + device conversion", "device: conversion in place"};
+      static const char *const out_name[] = {"pageable: staged", "pinned: DMA", "device: written in place"};
       for (size_t l = 0; l < nworkers; l++)
         fprintf(stderr, "[piplib-b200] device %d lane %zu: plan %.3f convert %.3f run %.3f emit %.3f s\n", devices[l / lanes], l % lanes,
                 tstage[l * 4], tstage[l * 4 + 1], tstage[l * 4 + 2], tstage[l * 4 + 3]);
       fprintf(stderr, "[piplib-b200] total %.3f s, %zu chunks, %zu devices x %zu lanes (%zu of them convert on the host), pool %u, input %s, output %s\n",
-              wall() - t0, nchunks, devices.size(), lanes, in_pinned ? host_lanes : lanes, host_threads(),
-              in_pinned ? "pinned: DMA + device conversion" : "pageable: host conversion",
-              out_pinned ? "pinned: DMA" : "pageable: staged");
+              wall() - t0, nchunks, devices.size(), lanes, in_route == IN_DMA_CONVERT ? host_lanes : in_route == IN_HOST_CONVERT ? lanes : 0,
+              host_threads(), in_name[in_route], out_name[out_route]);
     }
     PipBatchStats_dp acc;
     memset(&acc, 0, sizeof acc);

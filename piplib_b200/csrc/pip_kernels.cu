@@ -538,6 +538,34 @@ extern "C" cudaError_t pip_launch_convert(const PipConvertArgs *A, int elem_log2
   return cudaGetLastError();
 }
 
+/* ---- caller arrays in device memory (pip_solve_dense_dp): a chunk's per-problem results, written where the
+ * caller keeps them.  The same mapping the host applies to a staged chunk: a status that is not final becomes
+ * PIP_ST_CAPACITY, a span is the chunk's base plus the problem's slot offset, a length loses its narrow flag. */
+__global__ void __launch_bounds__(256) pip_emit_device_kernel(const int *st, const pip_u64 *hs, const long long *off,
+                                                              const long long *len, long long n, long long base,
+                                                              int *status, pip_u64 *hashes, long long *ser_off,
+                                                              long long *ser_len)
+{
+  const long long i0 = (long long)blockIdx.x * blockDim.x + threadIdx.x, step = (long long)gridDim.x * blockDim.x;
+  for (long long i = i0; i < n; i += step) {
+    const int s0 = st[i];
+    status[i] = PIP_STATUS_IS_FINAL(s0) ? s0 : PIP_ST_CAPACITY;
+    if (hashes) hashes[i] = hs[i];
+    if (ser_off) ser_off[i] = base + off[i];
+    if (ser_len) ser_len[i] = len[i] & ~PIP_LEN_NARROW;
+  }
+}
+extern "C" cudaError_t pip_launch_emit_device(const int *st, const pip_u64 *hs, const long long *off, const long long *len,
+                                              long long n, long long base, int *status, pip_u64 *hashes,
+                                              long long *ser_off, long long *ser_len, cudaStream_t stream)
+{
+  long long blocks = (n + 255) / 256;
+  if (blocks > 148 * 8) blocks = 148 * 8;
+  if (blocks < 1) blocks = 1;
+  pip_emit_device_kernel<<<(int)blocks, 256, 0, stream>>>(st, hs, off, len, n, base, status, hashes, ser_off, ser_len);
+  return cudaGetLastError();
+}
+
 /* single-CTA exclusive scan of ncells (n up to a few million: 1024 threads, chunked) */
 __global__ void pip_scan_kernel(const PipResult *res, const int *order, long long *dst_off, int nprob, long long *total,
                                 int ser_mode)

@@ -31,6 +31,11 @@ cudaError_t pip_launch_gather_words(PipResult *res, const int *order, const PipC
                                     cudaStream_t stream);
 cudaError_t pip_launch_init_results(PipResult *res, long long n, cudaStream_t stream);
 cudaError_t pip_launch_convert(const PipConvertArgs *A, int elem_log2, cudaStream_t stream);
+/* a stream_out chunk's per-problem arrays (PipDeviceOut) -> the caller's device arrays at the chunk's first problem;
+ * hashes / ser_off / ser_len may be NULL */
+cudaError_t pip_launch_emit_device(const int *st, const pip_u64 *hs, const long long *off, const long long *len,
+                                   long long n, long long base, int *status, pip_u64 *hashes,
+                                   long long *ser_off, long long *ser_len, cudaStream_t stream);
 cudaError_t pip_launch_image(const PipProblem *prob, const void *pool, int elem_log2, long long n, const PipLayout *lay,
                              pip_i64 *images, int image_words, int image_w1, int vbytes, cudaStream_t stream);
 int pip_layout_compute(int nvar, int nparm, int ni, int nc, int flags, int level, int words, int vbytes, PipLayout *out);
