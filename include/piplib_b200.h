@@ -15,6 +15,8 @@
  *                             cells or a hash per problem.  This is the bulk path used by
  *                             bench.py (host buffers in, host buffers out); it also reads and
  *                             writes caller arrays in device memory.
+ *   pip_solve_dense_info_dp   pip_solve_dense_dp plus a per-problem report: the int64 overflow flag and the
+ *                             pivot, cut and split counts (PipProblemInfo_dp).
  *   pip_device_*              the same batch with inputs/outputs resident in device memory
  *                             (kernel-only timing; pointers are CUdeviceptr values as integers).
  *   pip_quast_serialize_dp    PipQuast -> int64 stream (test/interop helper).
@@ -130,6 +132,37 @@ int pip_solve_dense_dp(long long n, int dom_rows, int dom_cols, const long long 
                        int *status, unsigned long long *hashes,
                        long long *ser, long long ser_cap, long long *ser_off, long long *ser_len);
 
+/* Per-problem solve report of a dense batch.  Each field equals, problem for problem, the field of the
+ * oracle's per-problem statistics (oracle/pyoracle.py PortStats, oracle/pip_oracle.c) named beside it: */
+typedef struct {
+  unsigned flags;           /* wrapped > 0: PIP_FLAG_WRAPPED (bit 0), as pip_last_batch_flags_dp reports it: an exact
+                               128-bit product of a pivot update left int64 (see PipBatchStats_dp.wrapped).  The
+                               whole-grid class (non-parametric problems that outgrow the team classes) does not
+                               detect the wrap: a problem it solves reports 0, there and in PipBatchStats_dp.wrapped */
+  unsigned pivots;          /* pivots: successful pivots, those of compa_test / context feasibility sub-solves included */
+  unsigned cuts;            /* cuts_const + cuts_parm: Gomory cuts, constant and parametric */
+  unsigned splits;          /* splits: parametric splits (If nodes emitted by the main solve) */
+  unsigned max_rows;        /* max_rows: the largest nligne (unknowns + rows) of a pivot */
+  unsigned max_cols;        /* max_cols: the largest ncol of a pivot */
+  unsigned spare[2];        /* zero */
+} PipProblemInfo_dp;        /* 32 bytes */
+
+/* pip_solve_dense_dp, and the report of problem i in info[i] (NULL: none; pip_solve_dense_dp is this call with
+ * info = NULL).  info is an output like status / hashes / ser: host or device memory, placed with the other
+ * outputs (a device-resident info beside host outputs, or the reverse, returns -3 before anything is written).
+ * The record belongs to the attempt that gave the final status: a problem re-run one size class up, handed over
+ * to the cooperative launch or to the whole-grid class reports that last run only; under subtree donation it is
+ * the sum over the problem's segments up to the verdict.  For a fatal status (1000+c, 2000) the counters are those
+ * at the verdict (a cell-limit verdict, 1026, met inside a donated subtree cannot be placed in it: such a problem
+ * is solved once more without donation); for 4001 / 4002 the record is all zero.  Same return codes as
+ * pip_solve_dense_dp. */
+int pip_solve_dense_info_dp(long long n, int dom_rows, int dom_cols, const long long *dom,
+                            int has_ctx, int ctx_rows, int ctx_cols, const long long *ctx,
+                            int bignum, const PipOptions_dp *options,
+                            int *status, unsigned long long *hashes,
+                            long long *ser, long long ser_cap, long long *ser_off, long long *ser_len,
+                            PipProblemInfo_dp *info);
+
 /* Page-lock a caller buffer (cudaHostRegister, visible to every device) so that pip_solve_dense_dp moves
  * it by DMA alone: input arrays `dom` / `ctx` registered this way are uploaded as they are and converted to
  * tableaus on the device (tab_Matrix2Tableau_xx, source/tab.c:292-393, as a kernel); an output stream
@@ -164,6 +197,10 @@ int pip_device_batch_run(pip_device_batch *b, int fetch_cells, float *device_ms)
 /* results of the last run: status always; hashes if that run decoded on the device (fetch_cells = 0) or fetched the cells.
  * They are read out of the engines' buffers in HBM: call it before the next solve on the same device. */
 int pip_device_batch_results(pip_device_batch *b, int *status, unsigned long long *hashes);
+/* the per-problem reports of the last run (PipProblemInfo_dp, n records) into a host array; read like the results.
+ * A run that decodes on the device (fetch_cells = 0) writes them only when they were asked for: info = NULL makes
+ * every later run of b write them (returns 0); the reports of a run that did not write them return -3. */
+int pip_device_batch_info(pip_device_batch *b, PipProblemInfo_dp *info);
 void pip_device_batch_destroy(pip_device_batch *b);
 
 /* One LARGE non-parametric tableau solved by the whole grid (BASELINE config 4; the tableau lives

@@ -10,7 +10,7 @@ import os
 
 import numpy as np
 
-from .ctypes_defs import CELL_DTYPE
+from .ctypes_defs import CELL_DTYPE, INFO_DTYPE
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("PIPLIB_B200_LIB") or os.path.join(HERE, "lib", "libpiplib_dp.so")
@@ -73,11 +73,14 @@ def lib():
         L.pip_quast_print_dp.argtypes = [C.c_void_p, C.c_void_p, C.c_int]
         L.pip_traiter_batch_dp.restype = C.c_int
         L.pip_solve_dense_dp.restype = C.c_int
+        L.pip_solve_dense_info_dp.restype = C.c_int
         L.pip_device_batch_create.restype = C.c_void_p
         L.pip_device_batch_run.restype = C.c_int
         L.pip_device_batch_run.argtypes = [C.c_void_p, C.c_int, C.POINTER(C.c_float)]
         L.pip_device_batch_results.restype = C.c_int
         L.pip_device_batch_results.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p]
+        L.pip_device_batch_info.restype = C.c_int
+        L.pip_device_batch_info.argtypes = [C.c_void_p, C.c_void_p]
         L.pip_device_batch_destroy.argtypes = [C.c_void_p]
         L.pip_large_create_dp.restype = C.c_void_p
         L.pip_large_run_dp.restype = C.c_int
@@ -338,6 +341,9 @@ class _HostArrays:
     def zeros(self, n, dtype):
         return np.zeros(n, dtype=np.uint64 if dtype == "u64" else dtype)
 
+    def info(self, n):
+        return np.zeros(n, dtype=INFO_DTYPE)
+
     def empty(self, n):
         return np.empty(n, dtype=np.int64)
 
@@ -358,15 +364,22 @@ class _CudaTensors:
     def zeros(self, n, dtype):
         return self.torch.zeros(n, dtype=self.torch.int32 if dtype == np.int32 else self.torch.int64, device=self.device)
 
+    def info(self, n):
+        return self.torch.zeros((n, 8), dtype=self.torch.int32, device=self.device)
+
     def empty(self, n):
         return self.torch.empty(n, dtype=self.torch.int64, device=self.device)
 
 
-def solve_dense(dom, ctx, bignum=-1, want_hashes=True, want_ser=False, ser_cap_hint=None, out=None, **opts):
+def solve_dense(dom, ctx, bignum=-1, want_hashes=True, want_ser=False, ser_cap_hint=None, out=None, want_info=False,
+                **opts):
     """dom: [n, rows, cols] int64; ctx: [n, rows, cols] or None.  Host arrays (numpy), or torch CUDA tensors:
     these are read and the results written in GPU memory, and the results are CUDA tensors (status int32,
     hashes / ser / ser_off / ser_len int64; hashes hold the uint64 bits).
-    Returns dict(status, hashes, ser, ser_off, ser_len)."""
+    want_info=True adds the per-problem solve report (PipProblemInfo_dp: the overflow flag, pivots, cuts,
+    splits, largest tableau): a numpy array of INFO_DTYPE, or an int32 CUDA tensor [n, 8] holding the uint32
+    bits of flags, pivots, cuts, splits, max_rows, max_cols and the two spare words, in that order.
+    Returns dict(status, hashes, ser, ser_off, ser_len), and info when asked for."""
     L = lib()
     B = _CudaTensors(dom) if getattr(dom, "is_cuda", False) else _HostArrays()
     dom = B.input(dom)
@@ -384,6 +397,9 @@ def solve_dense(dom, ctx, bignum=-1, want_hashes=True, want_ser=False, ser_cap_h
     hashes = None
     if want_hashes:
         hashes = out["hashes"] if reuse and out.get("hashes") is not None else B.zeros(n, "u64")
+    info = None
+    if want_info:
+        info = out["info"] if reuse and out.get("info") is not None else B.info(n)
     o = make_options(**opts)
     ser = ser_off = ser_len = None
     cap = 0
@@ -397,14 +413,11 @@ def solve_dense(dom, ctx, bignum=-1, want_hashes=True, want_ser=False, ser_cap_h
             cap = (ser_cap_hint or 448) * n + 1024
             ser = B.empty(cap)
     while True:
-        _ready(dom, ctx, status, hashes, ser, ser_off, ser_len)
-        rc = L.pip_solve_dense_dp(C.c_longlong(n), dr, dc, _ptr(dom), has, cr, cc, cp,
-                                  int(bignum), C.byref(o), _ptr(status),
-                                  _ptr(hashes) if want_hashes else None,
-                                  _ptr(ser) if want_ser else None,
-                                  C.c_longlong(cap),
-                                  _ptr(ser_off) if want_ser else None,
-                                  _ptr(ser_len) if want_ser else None)
+        _ready(dom, ctx, status, hashes, ser, ser_off, ser_len, info)
+        args = (C.c_longlong(n), dr, dc, _ptr(dom), has, cr, cc, cp, int(bignum), C.byref(o), _ptr(status),
+                _ptr(hashes) if want_hashes else None, _ptr(ser) if want_ser else None, C.c_longlong(cap),
+                _ptr(ser_off) if want_ser else None, _ptr(ser_len) if want_ser else None)
+        rc = L.pip_solve_dense_info_dp(*args, _ptr(info)) if want_info else L.pip_solve_dense_dp(*args)
         if rc == -2:
             was_pinned = reuse and out.get("ser") is ser and isinstance(ser, np.ndarray)
             cap = int(ser_off[n]) + 16
@@ -418,7 +431,10 @@ def solve_dense(dom, ctx, bignum=-1, want_hashes=True, want_ser=False, ser_cap_h
         if rc != 0:
             raise RuntimeError("pip_solve_dense_dp failed: %d" % rc)
         break
-    return dict(status=status, hashes=hashes, ser=ser, ser_off=ser_off, ser_len=ser_len)
+    r = dict(status=status, hashes=hashes, ser=ser, ser_off=ser_off, ser_len=ser_len)
+    if want_info:
+        r["info"] = info
+    return r
 
 
 def alloc_result(n, words_per_problem=448, pinned=False):
@@ -467,6 +483,20 @@ class DeviceBatch:
         if rc != 0:
             raise RuntimeError("pip_device_batch_results failed: %d" % rc)
         return status, hashes
+
+    def keep_info(self):
+        """make every later run() write the per-problem solve reports (a run on the device writes none unless asked)"""
+        if lib().pip_device_batch_info(self.h, None) != 0:
+            raise RuntimeError("pip_device_batch_info failed")
+
+    def info(self):
+        """the per-problem solve reports of the last run (numpy array of INFO_DTYPE); raises if that run wrote none
+        (see keep_info)"""
+        out = np.zeros(self.n, dtype=INFO_DTYPE)
+        rc = lib().pip_device_batch_info(self.h, out.ctypes.data_as(C.c_void_p))
+        if rc != 0:
+            raise RuntimeError("pip_device_batch_info failed: %d" % rc)
+        return out
 
     def close(self):
         if self.h:

@@ -94,6 +94,7 @@ struct PipEngine::Impl {
   cudaEvent_t ev0 = nullptr, ev1 = nullptr;
   DevBuf d_prob, d_pool, d_res, d_cells, d_stack, d_gwork, d_queue, d_order, d_off, d_compact, d_total, d_prof, d_parm, d_hash;
   DevBuf d_so_status, d_so_hash, d_so_off, d_so_len, d_so_ctl;     /* stream_out: per-problem arrays, control + stats */
+  DevBuf d_so_info;                /* stream_out: per-problem reports, when asked for */
   DevBuf d_image;                  /* arena images of a uniform batch (pip_image_kernel) */
   DevBuf d_stl_offers, d_stl_segs, d_stl_next, d_stl_hwm, d_stl_head_next, d_stl_head_hwm, d_stl_ctl;   /* subtree donation */
   DevBuf d_heavy;                /* problems handed over to the donation launch */
@@ -322,6 +323,12 @@ void PipEngine::run(const PipBatchIn &in, PipBatchOut &out)
     so.words64 = in.words64 ? 1 : 0;
     so.status = (int *)E.d_so_status.p; so.hash = (pip_u64 *)E.d_so_hash.p;
     so.off = (long long *)E.d_so_off.p; so.len = (long long *)E.d_so_len.p;
+    if (in.want_info) {
+      /* every problem's report is written by the decode pass of each round it takes part in (the last one wins) */
+      E.d_so_info.reserve(n * sizeof(PipInfo));
+      CK(cudaMemsetAsync(E.d_so_info.p, 0, n * sizeof(PipInfo), s));
+      so.info = (PipInfo *)E.d_so_info.p;
+    }
   }
   E.d_queue.reserve(64);
   E.d_prof.reserve(sizeof(unsigned long long) * PIP_NPHASE);
@@ -392,6 +399,9 @@ void PipEngine::run(const PipBatchIn &in, PipBatchOut &out)
   size_t open_total = n;                /* problems not final yet, all classes */
   for (int k = -2; k < N_G && open_total; k++) {
     int last_open = -1;                 /* problems of this class still open after the previous attempt */
+    /* with the reports, problems left open by an attempt with subtree donation (a cell-limit verdict met inside a
+     * donated subtree, pip_gather_words_kernel) are solved again without it: that attempt may retire none */
+    bool plain = false, redo = false;
     for (int attempt = 0;; attempt++) {
       order.clear();
       for (size_t i = 0; i < n; i++) if (cls[i] == k) order.push_back((int)i);
@@ -399,7 +409,7 @@ void PipEngine::run(const PipBatchIn &in, PipBatchOut &out)
       const int m = (int)order.size();
       /* every attempt must retire at least one problem (a warp always has room for one worst-case
        * solution): anything else is a scheduling bug, never a verdict */
-      if (last_open >= 0 && m >= last_open)
+      if (last_open >= 0 && m >= last_open && !redo)
         throw std::runtime_error("piplib-b200: size class made no progress (" + std::to_string(m) + " problems open)");
       last_open = m;
       const bool identity = (size_t)m == n;           /* every problem of the batch: no permutation needed */
@@ -516,6 +526,7 @@ void PipEngine::run(const PipBatchIn &in, PipBatchOut &out)
       bool steal = words_round && k < 0 &&
                    (dmode > 0 || (dmode < 0 && (long long)m <= 2ll * cs.warps && (!in.uniform || in.uniform->nparm > 0)));
       if (const char *sv = getenv("PIPLIB_B200_STEAL")) steal = words_round && k < 0 && atoi(sv) != 0;
+      steal = steal && !plain;
       auto arm_donation = [&](PipSteal &S) {
         S.mode = 1; S.cap = 1 << 16;
         if (const char *cv = getenv("PIPLIB_B200_STEAL_CAP")) S.cap = std::max(1024, atoi(cv));
@@ -546,6 +557,8 @@ void PipEngine::run(const PipBatchIn &in, PipBatchOut &out)
         heavy_budget = (unsigned)atoi(hv);
         handover = words_round && k < 0 && !steal && heavy_budget > 0;
       }
+      handover = handover && !plain;
+      redo = false;
       PipLaunch L2;
       const PipSteal *gather_stl = steal ? &L.steal : nullptr;
       if (handover) {
@@ -704,13 +717,14 @@ void PipEngine::run(const PipBatchIn &in, PipBatchOut &out)
                 round - 1, k, attempt, m, cs.warps, (int)cs.words, t_round, escalated + pending, pending, use_large ? " [whole-grid kernel]" : "",
                 team_smem ? " [team arena in shared memory]" : "");
       if (pending == 0) break;
+      if (in.want_info && stream_out && (steal || handover) && !plain) plain = redo = true;
     }
   }
   CK(cudaEventElapsedTime(&out.times.device_ms, E.ev0, E.ev1));
   if (stream_out) {
     out.dev.words = (const pip_i64 *)E.d_compact.p;
     out.dev.slots = slots_done;
-    out.dev.status = so.status; out.dev.hash = so.hash; out.dev.off = so.off; out.dev.len = so.len;
+    out.dev.status = so.status; out.dev.hash = so.hash; out.dev.off = so.off; out.dev.len = so.len; out.dev.info = so.info;
     for (int k = 0; k < PIP_SO_NSTAT; k++) out.dev.stats[k] = h_ctl[PIP_SO_NCTL + k];
     /* anything still unsolved is too large for the ladder: its status array entry says CAPACITY already
      * (the last decode pass wrote the record's status) */

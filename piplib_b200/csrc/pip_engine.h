@@ -30,6 +30,7 @@ struct PipBatchIn {
                                            arrays stay on the device (PipBatchOut::dev), nothing per problem
                                            crosses PCIe inside run() unless a problem has to change class */
   bool words64 = false;                 /* stream_out: every word as int64 (else int32 where it fits) */
+  bool want_info = false;               /* stream_out: write the per-problem reports (PipDeviceOut::info) */
   bool overlapped = false;              /* other engine lanes run beside this batch: its tail is not idle time (no hand-over) */
   long long words_hint = 0;             /* stream_out: expected 64-bit slots for the whole batch (0 = default) */
   /* called when a problem's input does not fit the int32 pool (PIP_F_WIDE_INPUT): returns the int64 pool */
@@ -44,6 +45,7 @@ struct PipDeviceOut {
   const int *status = nullptr;
   const pip_u64 *hash = nullptr;
   const long long *off = nullptr, *len = nullptr;   /* per problem: slot offset, words | PIP_LEN_NARROW */
+  const PipInfo *info = nullptr;        /* per problem: the report (PipBatchIn::want_info), else NULL */
   unsigned long long stats[PIP_SO_NSTAT] = {0};   /* pivots, cuts, subsolves, splits, elem_updates, cells, max_rows, max_cols, wrapped */
 };
 

@@ -34,8 +34,12 @@
 #include "pip_decode.h"
 #include "pip_engine.h"
 #include "pip_kernels.h"
+#include "pip_segments.h"
 
 typedef long long I;
+
+static_assert(sizeof(PipProblemInfo_dp) == 32 && sizeof(PipInfo) == sizeof(PipProblemInfo_dp), "report layouts must agree");
+static_assert(PIP_INFO_FLAG_WRAPPED == PIP_FLAG_WRAPPED, "report flags must agree");
 
 namespace {
 
@@ -1060,12 +1064,13 @@ long long len_quast(const C &c, int *i, int Bg, int Urs_p, int flags)
  * pass 2 decodes in place, hashing on the fly. */
 void emit_chunk(const DenseArgs &A, DenseChunk &C, int *status, unsigned long long *hashes,
                 long long *ser, long long ser_cap, long long *ser_off, long long *ser_len,
-                std::atomic<long long> *cursor, size_t nthreads)
+                std::atomic<long long> *cursor, size_t nthreads, PipInfo *info = nullptr)
 {
   const size_t n = C.n;
   const bool keep = ser != nullptr && ser_off != nullptr;
   const int simplify = A.opt.Simplify;
   for (size_t i = 0; i < n; i++) status[C.first + i] = C.out.res[i].status;
+  if (info) for (size_t i = 0; i < n; i++) info[C.first + i] = pip_info_of(C.out.res[i]);
   if (!keep && !hashes) return;
   C.words.assign(n, 0);
   nthreads = std::max<size_t>(1, std::min(nthreads, (n + 63) / 64));
@@ -1250,7 +1255,19 @@ int pip_solve_dense_dp(long long n, int dom_rows, int dom_cols, const long long 
                        int *status, unsigned long long *hashes,
                        long long *ser, long long ser_cap, long long *ser_off, long long *ser_len)
 {
+  return pip_solve_dense_info_dp(n, dom_rows, dom_cols, dom, has_ctx, ctx_rows, ctx_cols, ctx, bignum, options,
+                                 status, hashes, ser, ser_cap, ser_off, ser_len, nullptr);
+}
+
+int pip_solve_dense_info_dp(long long n, int dom_rows, int dom_cols, const long long *dom,
+                            int has_ctx, int ctx_rows, int ctx_cols, const long long *ctx,
+                            int bignum, const PipOptions_dp *options,
+                            int *status, unsigned long long *hashes,
+                            long long *ser, long long ser_cap, long long *ser_off, long long *ser_len,
+                            PipProblemInfo_dp *info_out)
+{
   if (n <= 0) return 0;
+  PipInfo *const info = (PipInfo *)info_out;
   std::lock_guard<std::mutex> dense_guard(g_dense_mu);
   KeepCurrentDevice keep_device;
   try {
@@ -1273,7 +1290,8 @@ int pip_solve_dense_dp(long long n, int dom_rows, int dom_cols, const long long 
     const bool in_device = on_device(dom);
     const bool ctx_device = ctx_used && on_device(ctx);
     int nout = 0, nout_device = 0;
-    for (const void *p : {(const void *)status, (const void *)hashes, (const void *)ser, (const void *)ser_off, (const void *)ser_len})
+    for (const void *p : {(const void *)status, (const void *)hashes, (const void *)ser, (const void *)ser_off, (const void *)ser_len,
+                          (const void *)info})
       if (p) { nout++; nout_device += on_device(p) ? 1 : 0; }
     const bool out_device = nout_device > 0;
     const bool host_decoder = A.opt.Simplify || (A.opt.Compute_dual && !A.opt.Nq);
@@ -1468,6 +1486,7 @@ int pip_solve_dense_dp(long long n, int dom_rows, int dom_cols, const long long 
             /* other lanes keep the machine busy during this chunk's tail -- except at the end of the call */
             in.overlapped = nworkers > 1 && c + tail_chunks < nchunks;
             in.words64 = out_route == OUT_PINNED_DMA || (out_route == OUT_DEVICE && keep);
+            in.want_info = info != nullptr;
           }
           double td = wall();
           E.run(in, C.out);
@@ -1483,22 +1502,25 @@ int pip_solve_dense_dp(long long n, int dom_rows, int dom_cols, const long long 
                 if (D.slots && base + D.slots <= ser_cap)
                   pip_cuda_check(cudaMemcpyAsync(ser + base, D.words, (size_t)D.slots * 8, cudaMemcpyDeviceToDevice, s), "D2D quasts");
               }
-              pip_cuda_check(pip_launch_emit_device(D.status, D.hash, D.off, D.len, (long long)cn, base, status + C.first,
+              pip_cuda_check(pip_launch_emit_device(D.status, D.hash, D.off, D.len, D.info, (long long)cn, base, status + C.first,
                                                     hashes ? hashes + C.first : nullptr,
                                                     keep ? ser_off + C.first : nullptr,
-                                                    keep && ser_len ? ser_len + C.first : nullptr, s), "emit kernel");
+                                                    keep && ser_len ? ser_len + C.first : nullptr,
+                                                    info ? info + C.first : nullptr, s), "emit kernel");
               pip_cuda_check(cudaStreamSynchronize(s), "sync after emit");
             } else {
               /* per-problem arrays: SoA on the device -> pinned scratch -> the caller's arrays */
-              const size_t soa = cn * (sizeof(int) + sizeof(pip_u64) + 2 * sizeof(long long));
+              const size_t soa = cn * (sizeof(int) + sizeof(pip_u64) + 2 * sizeof(long long) + (info ? sizeof(PipInfo) : 0));
               unsigned char *hp = (unsigned char *)E.pinned_scratch(1, soa + 64);
               long long *h_off = (long long *)hp, *h_len = h_off + cn;
               pip_u64 *h_hash = (pip_u64 *)(h_len + cn);
-              int *h_st = (int *)(h_hash + cn);
+              PipInfo *h_info = (PipInfo *)(h_hash + cn);
+              int *h_st = (int *)(h_info + (info ? cn : 0));
               std::unique_lock<std::mutex> link(g_d2h_mu[device]);
               pip_cuda_check(cudaMemcpyAsync(h_off, D.off, cn * 8, cudaMemcpyDeviceToHost, s), "D2H offsets");
               pip_cuda_check(cudaMemcpyAsync(h_len, D.len, cn * 8, cudaMemcpyDeviceToHost, s), "D2H lengths");
               pip_cuda_check(cudaMemcpyAsync(h_hash, D.hash, cn * 8, cudaMemcpyDeviceToHost, s), "D2H hashes");
+              if (info) pip_cuda_check(cudaMemcpyAsync(h_info, D.info, cn * sizeof(PipInfo), cudaMemcpyDeviceToHost, s), "D2H reports");
               pip_cuda_check(cudaMemcpyAsync(h_st, D.status, cn * 4, cudaMemcpyDeviceToHost, s), "D2H statuses");
               lane_stats[w].d2h_bytes += soa;
               if (out_route == OUT_PINNED_DMA) {
@@ -1519,6 +1541,7 @@ int pip_solve_dense_dp(long long n, int dom_rows, int dom_cols, const long long 
                   if (ser_len) ser_len[C.first + i] = h_len[i] & ~PIP_LEN_NARROW;
                 }
                 if (hashes) memcpy(hashes + C.first, h_hash, cn * 8);
+                if (info) memcpy(info + C.first, h_info, cn * sizeof(PipInfo));   /* (not final: all zero already) */
               } else {
                 pip_i64 *h_words = nullptr;
                 if (keep && D.slots) {
@@ -1530,13 +1553,14 @@ int pip_solve_dense_dp(long long n, int dom_rows, int dom_cols, const long long 
                 link.unlock();
                 emit_chunk_staged(C.first, cn, h_words, h_st, h_hash, h_off, h_len, status, hashes, ser, ser_cap, ser_off,
                                   ser_len, &cursor, nthreads, at);
+                if (info) memcpy(info + C.first, h_info, cn * sizeof(PipInfo));
               }
             }
             PipBatchStats_dp &ls = lane_stats[w];
             ls.pivots += D.stats[0]; ls.cuts += D.stats[1]; ls.subsolves += D.stats[2]; ls.splits += D.stats[3];
             ls.elem_updates += D.stats[4]; ls.cells += D.stats[5]; ls.wrapped += D.stats[8];
             ls.max_rows = std::max(ls.max_rows, (unsigned)D.stats[6]); ls.max_cols = std::max(ls.max_cols, (unsigned)D.stats[7]);
-          } else emit_chunk(A, C, status, hashes, ser, ser_cap, ser_off, ser_len, &cursor, nthreads);
+          } else emit_chunk(A, C, status, hashes, ser, ser_cap, ser_off, ser_len, &cursor, nthreads, info);
           tstage[w * 4 + 2] += te - td; tstage[w * 4 + 3] += wall() - te;
           accumulate(lane_stats[w], C.out);
           if (timing)
@@ -1592,6 +1616,7 @@ struct pip_device_batch {
   bool fetched = false;
   bool device_decode = false;           /* run() = solve + decode on the device (serialised quasts stay in HBM) */
   bool uniform = false;
+  bool keep_info = false;               /* runs write the per-problem reports (pip_device_batch_info(b, NULL)) */
   PipProblem shape;
   std::vector<PipDecodeParm> parm;
   int device = 0;
@@ -1652,6 +1677,7 @@ int pip_device_batch_run(pip_device_batch *b, int fetch_cells, float *device_ms)
     if (stream) {
       if (b->uniform) in.uniform_decode = &b->parm[0]; else in.h_decode = b->parm.data();
       in.stream_out = true;
+      in.want_info = b->keep_info;
     } else in.fetch_cells = fetch_cells != 0;
     b->parts.clear();
     /* A launch ends with its heaviest problems, one warp each, on an idle machine (loop nests: the last ~12 ms
@@ -1789,6 +1815,34 @@ int pip_device_batch_results(pip_device_batch *b, int *status, unsigned long lon
   if (hashes && !b->fetched) return -3;
   if (hashes) emit_chunk(b->A, b->C, status, hashes, nullptr, 0, nullptr, nullptr, nullptr, host_threads());
   else for (size_t i = 0; i < b->C.n; i++) status[i] = b->C.out.res[i].status;
+  return 0;
+}
+
+int pip_device_batch_info(pip_device_batch *b, PipProblemInfo_dp *info_out)
+{
+  PipInfo *const info = (PipInfo *)info_out;
+  if (!info) { b->keep_info = true; return 0; }
+  try {
+    if (!b->parts.empty()) {             /* last run went in parts: every lane holds its part's reports */
+      for (auto &P : b->parts) if (!P.out.dev.info) return -3;
+      pip_cuda_check(cudaSetDevice(b->device), "cudaSetDevice");
+      for (auto &P : b->parts)
+        pip_cuda_check(cudaMemcpy(info + P.first, P.out.dev.info, P.n * sizeof(PipInfo), cudaMemcpyDeviceToHost), "D2H reports");
+      return 0;
+    }
+    const PipDeviceOut &D = b->C.out.dev;
+    if (D.status) {                      /* last run decoded on the device */
+      if (!D.info) return -3;
+      pip_cuda_check(cudaSetDevice(b->device), "cudaSetDevice");
+      pip_cuda_check(cudaMemcpy(info, D.info, b->C.n * sizeof(PipInfo), cudaMemcpyDeviceToHost), "D2H reports");
+      return 0;
+    }
+    if (b->C.out.res.size() != b->C.n) return -1;
+    for (size_t i = 0; i < b->C.n; i++) info[i] = pip_info_of(b->C.out.res[i]);
+  } catch (const std::exception &e) {
+    fprintf(stderr, "%s\n", e.what());
+    return -1;
+  }
   return 0;
 }
 

@@ -296,6 +296,7 @@ pip_serialize_warp_kernel(PipResult *res, const int *order, const PipCell *cells
         so.hash[p] = h;
         so.off[p] = base;
         so.len[p] = has_words ? ((long long)r.ser_words | (narrow ? PIP_LEN_NARROW : 0ll)) : 0ll;
+        if (so.info) so.info[p] = pip_info_of(r);
       } else {
         res[p].cell_off = base;
         if (hashes) hashes[p] = h;
@@ -373,6 +374,9 @@ pip_gather_words_kernel(PipResult *res, const int *order, const PipCell *cells, 
       r.elem_updates_lo = (unsigned)(R.elem_updates & 0xffffffffull); r.elem_updates_hi = (unsigned)(R.elem_updates >> 32);
       r.max_rows = R.max_rows; r.max_cols = R.max_cols;
       r.rflags = (R.any_flags_or & ~PIP_RES_SER32) | (R.all_flags_and & PIP_RES_SER32);
+      /* the reports ask for the counters at the verdict, and a cell limit met inside a donated segment has none
+       * (pip_segments.h): such a problem goes back to the ladder, which solves it again without donation */
+      if (so.info && r.status == PIP_ST_FATAL + 26 && R.verdict_seg >= 0) r.status = PIP_ST_PENDING;
       if (lane == 0) res[p].status = r.status;         /* the ladder reads the resolved verdict */
     }
     const bool has_words = r.status == PIP_ST_OK || r.status == PIP_ST_VOID;
@@ -413,6 +417,7 @@ pip_gather_words_kernel(PipResult *res, const int *order, const PipCell *cells, 
       so.hash[p] = has_words ? h + PIP_HASH_INIT : 0ull;
       so.off[p] = base;
       so.len[p] = nw | (narrow && nw ? PIP_LEN_NARROW : 0ll);
+      if (so.info) so.info[p] = pip_info_of(r);
     }
     if (PIP_STATUS_IS_FINAL(r.status)) {
       finals++;
@@ -540,29 +545,36 @@ extern "C" cudaError_t pip_launch_convert(const PipConvertArgs *A, int elem_log2
 
 /* ---- caller arrays in device memory (pip_solve_dense_dp): a chunk's per-problem results, written where the
  * caller keeps them.  The same mapping the host applies to a staged chunk: a status that is not final becomes
- * PIP_ST_CAPACITY, a span is the chunk's base plus the problem's slot offset, a length loses its narrow flag. */
+ * PIP_ST_CAPACITY (and its report all zero), a span is the chunk's base plus the problem's slot offset, a length
+ * loses its narrow flag. */
 __global__ void __launch_bounds__(256) pip_emit_device_kernel(const int *st, const pip_u64 *hs, const long long *off,
-                                                              const long long *len, long long n, long long base,
-                                                              int *status, pip_u64 *hashes, long long *ser_off,
-                                                              long long *ser_len)
+                                                              const long long *len, const PipInfo *inf, long long n,
+                                                              long long base, int *status, pip_u64 *hashes,
+                                                              long long *ser_off, long long *ser_len, PipInfo *info)
 {
   const long long i0 = (long long)blockIdx.x * blockDim.x + threadIdx.x, step = (long long)gridDim.x * blockDim.x;
   for (long long i = i0; i < n; i += step) {
     const int s0 = st[i];
-    status[i] = PIP_STATUS_IS_FINAL(s0) ? s0 : PIP_ST_CAPACITY;
+    const bool final = PIP_STATUS_IS_FINAL(s0);
+    status[i] = final ? s0 : PIP_ST_CAPACITY;
     if (hashes) hashes[i] = hs[i];
     if (ser_off) ser_off[i] = base + off[i];
     if (ser_len) ser_len[i] = len[i] & ~PIP_LEN_NARROW;
+    if (info) {
+      const PipInfo zero = {0, 0, 0, 0, 0, 0, {0, 0}};
+      info[i] = final ? inf[i] : zero;
+    }
   }
 }
 extern "C" cudaError_t pip_launch_emit_device(const int *st, const pip_u64 *hs, const long long *off, const long long *len,
-                                              long long n, long long base, int *status, pip_u64 *hashes,
-                                              long long *ser_off, long long *ser_len, cudaStream_t stream)
+                                              const PipInfo *inf, long long n, long long base, int *status, pip_u64 *hashes,
+                                              long long *ser_off, long long *ser_len, PipInfo *info, cudaStream_t stream)
 {
   long long blocks = (n + 255) / 256;
   if (blocks > 148 * 8) blocks = 148 * 8;
   if (blocks < 1) blocks = 1;
-  pip_emit_device_kernel<<<(int)blocks, 256, 0, stream>>>(st, hs, off, len, n, base, status, hashes, ser_off, ser_len);
+  pip_emit_device_kernel<<<(int)blocks, 256, 0, stream>>>(st, hs, off, len, inf, n, base, status, hashes, ser_off, ser_len,
+                                                          info);
   return cudaGetLastError();
 }
 

@@ -120,7 +120,15 @@ typedef struct {
   long long *len;                /* words; bit 62 set when they were written as int32 */
   unsigned long long *stats;     /* [PIP_SO_NSTAT]: pivots, cuts, subsolves, splits, elem_updates, cells, max_rows,
                                     max_cols, problems flagged PIP_RES_WRAPPED (final statuses only) */
+  struct PipInfo *info;          /* per-problem report (PipProblemInfo_dp) or NULL when the caller did not ask for it */
 } PipStreamOut;
+
+/* the per-problem report of the dense path, PipProblemInfo_dp of include/piplib_b200.h: the counters of the
+ * record a verdict came with; all zero for a status that is no verdict of the reference (4xxx) */
+typedef struct PipInfo {
+  unsigned flags, pivots, cuts, splits, max_rows, max_cols, spare[2];
+} PipInfo;
+#define PIP_INFO_FLAG_WRAPPED 1u         /* = PIP_FLAG_WRAPPED */
 #define PIP_LEN_NARROW (1ll << 62)
 #define PIP_SO_NSTAT 9
 enum { PIP_SO_SLOTS = 0, PIP_SO_FINALS = 1, PIP_SO_OVERFLOW = 2, PIP_SO_NCTL = 4 };

@@ -32,9 +32,13 @@ RESULT_DTYPE = np.dtype([("status", "i4"), ("ncells", "i4"), ("cell_off", "i8"),
                          ("max_cols", "u4"), ("ser_words", "u4"), ("elem_updates_lo", "u4"),
                          ("elem_updates_hi", "u4"), ("pad", "u4")])
 CELL_DTYPE = np.dtype([("kind", "i4"), ("pad", "i4"), ("p1", "i8"), ("p2", "i8")])
+# PipProblemInfo_dp (include/piplib_b200.h): the per-problem solve report of a dense batch
+INFO_DTYPE = np.dtype([("flags", "u4"), ("pivots", "u4"), ("cuts", "u4"), ("splits", "u4"), ("max_rows", "u4"),
+                       ("max_cols", "u4"), ("spare", "u4", (2,))])
 assert PROBLEM_DTYPE.itemsize == C.sizeof(PipProblem) == 32
 assert RESULT_DTYPE.itemsize == C.sizeof(PipResult) == 56
 assert CELL_DTYPE.itemsize == C.sizeof(PipCell) == 24
+assert INFO_DTYPE.itemsize == 32
 
 
 def pack_tableau_problems(cases):
